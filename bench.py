@@ -1,6 +1,6 @@
 """bench.py — ray-samples/s of the render_rays hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N ...        (one rank per GPU, NCCL)
 
 Workload (BASELINE.json configs[1] at N=1; configs[4]'s training shape at N>1 = the same 1024 rays
@@ -27,6 +27,11 @@ One JSON line on stdout (rank 0):
   image_800  configs[4] inference: one 800x800 view, contiguous ray shards + one all-gather.
 `--impl reference` times the unmodified reference (baseline/_ref, staged by tools/stage_reference.py)
 on the host cores; if it is absent, the numpy oracle port (oracle/) — `cpu_baseline.kind` says which.
+
+`--dump-outputs DIR` writes the six float32 result tensors of the last timed step (at N>1 also the
+all-gathered batch, `all_gather`) to DIR/<name>.npy.  The inputs are seeded, so two runs with the same
+arguments render the same rays with the same random numbers, and two builds can be compared output for output.
+The benchmark writes nothing into the repository tree.
 """
 import argparse
 import json
@@ -389,6 +394,8 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=dev)
     lib = _lib.load()
     K = args.steps
+    # randoms="kernel" seeds its draws from torch.initial_seed(): fixed, so that every run renders the same samples
+    torch.manual_seed(0)
 
     ws = [synthetic_weights(11), synthetic_weights(12)]   # random init: there are no checkpoints
     sd = [{k: torch.from_numpy(v) for k, v in w.items()} for w in ws]
@@ -498,7 +505,8 @@ def run_b200(args):
         if rank == 0:
             sampler.start()
         # ---- value: K steps, device-timed
-        run, graphed = timed_graph(lambda i: step(i), K)
+        last = {}                                       # the result tensors of the last step (graph-owned when graphed)
+        run, graphed = timed_graph(lambda i: last.update(step(i)) if i == K - 1 else step(i), K)
         for _ in range(2):
             run()                                       # graph warm-up replays (not timed)
         l0 = lib.nerfb200_launch_count()
@@ -506,6 +514,10 @@ def run_b200(args):
         launches = lib.nerfb200_launch_count() - l0
         if graphed:
             launches = K                               # replayed nodes do not pass through the library's counter
+        if args.dump_outputs and rank == 0:
+            if world > 1:
+                last["all_gather"] = gather_buf
+            dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in last.items()})
 
         # ---- kernel-only (roofline): the render kernel is the only node of a step (as in `value`: the uniform
         # numbers are Philox draws inside the kernel)
@@ -768,6 +780,23 @@ def _hard_exit(code, run_atexit=True, device=None):
     os._exit(code)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy (float32 or float64), so that two builds can be compared output
+    for output on the same seeded inputs."""
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{name}: dtype {a.dtype} is not float32 / float64")
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"outputs take {total} bytes, more than the {DUMP_LIMIT_BYTES} allowed")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _JSON_FD = None
 
 
@@ -784,6 +813,7 @@ def emit(obj):
 
 def main():
     global _JSON_FD
+    sys.dont_write_bytecode = True      # the project's modules are imported later; no __pycache__ in the tree
     sys.stdout.flush()
     _JSON_FD = os.dup(1)
     os.dup2(2, 1)
@@ -793,7 +823,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-train", action="store_true", help="skip the training-step leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result tensors of the last one to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -204,6 +204,50 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs_writes_float_arrays(tmp_path, monkeypatch):
+    """bench.py --dump-outputs writes float arrays as .npy and refuses other dtypes or more than its size limit
+    before writing anything."""
+    import numpy as np
+
+    import bench
+    a = {"rgb": np.arange(6, dtype=np.float32).reshape(2, 3), "depth": np.ones(2)}
+    bench.dump_outputs(str(tmp_path / "d"), a)
+    for k, v in a.items():
+        got = np.load(tmp_path / "d" / f"{k}.npy")
+        assert got.dtype == v.dtype and np.array_equal(got, v)
+    with pytest.raises(TypeError):
+        bench.dump_outputs(str(tmp_path / "i"), {"n": np.zeros(2, np.int32)})
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8)
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), a)
+    assert not (tmp_path / "i").exists() and not (tmp_path / "big").exists()
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_exactly(tmp_path):
+    """Two bench runs with the same arguments render the same inputs: their dumped last-step outputs are equal."""
+    import json
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, "bench.py", "--steps", "3", "--warmup", "3", "--no-train",
+                            "--dump-outputs", str(d)], cwd=ROOT, capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 3
+        dumps.append({p.stem: np.load(p) for p in sorted(d.glob("*.npy"))})
+    shapes = {"rgb_coarse": (1024, 3), "depth_coarse": (1024,), "opacity_coarse": (1024,),
+              "rgb_fine": (1024, 3), "depth_fine": (1024,), "opacity_fine": (1024,)}
+    assert {k: v.shape for k, v in dumps[0].items()} == shapes
+    for k, v in dumps[0].items():
+        assert v.dtype == np.float32 and np.isfinite(v).all(), k
+        assert np.array_equal(v, dumps[1][k]), k
+
+
 def test_integration_md_stub_matches_the_struct():
     """The ctypes stub printed in INTEGRATION.md section 4 is the struct the library takes (names, order, size)."""
     import re
