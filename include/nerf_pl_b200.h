@@ -144,6 +144,12 @@ size_t nerfb200_train_workspace_bytes(int64_t n_rays, int32_t n_samples, int32_t
  * counters and uploads the wgrad job table.  Synchronous with respect to `stream`. */
 int nerfb200_train_workspace_init(void* workspace, size_t bytes, int64_t n_rays, int32_t n_samples,
                                   int32_t n_importance, void* stream);
+/* fp16 gradient elements that the last nerfb200_render_backward on this workspace stored at the fp16
+ * limit (clipped by the saturating conversion) or as NaN, for the coarse and the fine pass: out[2] on
+ * the host.  0 unless a batch defeats the per-layer scale selection (DESIGN.md section 3); the weight
+ * gradients of a step with a non-zero count are inexact.  Synchronises `stream`. */
+int nerfb200_train_saturation(const void* workspace, int64_t n_rays, int32_t n_samples, int32_t n_importance,
+                              uint32_t* out, void* stream);
 typedef struct nerfb200_backward_args {
   const nerfb200_render_args* render;   /* as passed to the forward call */
   const float* const* params_coarse;    /* 24 device pointers */

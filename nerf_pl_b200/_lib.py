@@ -47,6 +47,7 @@ EXPORTS = [
     "nerfb200_train_workspace_bytes",
     "nerfb200_train_workspace_init",
     "nerfb200_render_backward",
+    "nerfb200_train_saturation",
     "nerfb200_adam_step",
     "nerfb200_generate_rays",
     "nerfb200_to_uint8",
@@ -185,6 +186,8 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.nerfb200_train_workspace_init.restype = c_int32
     lib.nerfb200_render_backward.argtypes = [POINTER(BackwardArgs), c_void_p]
     lib.nerfb200_render_backward.restype = c_int32
+    lib.nerfb200_train_saturation.argtypes = [c_void_p, c_int64, c_int32, c_int32, POINTER(ctypes.c_uint32), c_void_p]
+    lib.nerfb200_train_saturation.restype = c_int32
     lib.nerfb200_adam_step.argtypes = [c_int32, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p),
                                        POINTER(c_int64), c_float, c_float, c_float, c_float, c_float, c_int64, c_void_p]
     lib.nerfb200_adam_step.restype = c_int32

@@ -22,8 +22,9 @@
 // Per-sample gradients are fp16 with a power-of-two scale PER LAYER, chosen on the device in the
 // same step (no state carried between steps, deterministic): level 0 (dd) from a bound on its
 // largest element, |d rgb_pre|_max * max_n sum_c |W_rgb[c][n]|; levels 1..8 (dpre_8..dpre_1) from
-// the largest elements a PROBE pass of the chain kernel sees on one tile per SM (no stores), each
-// mapped to 64 (10 bits of headroom to the fp16 maximum, 20 bits of normal range below; gradients
+// that bound times the growth factor of each level, which a PROBE pass of the chain kernel measures on one
+// tile per SM (no stores; bwd_scale_kernel), each mapped to 64 (10 bits of headroom to the fp16 maximum,
+// 20 bits of normal range below; the real pass counts what still saturates; gradients
 // shrink or grow by orders of magnitude through 8 layers, one global scale costs precision in the
 // deep layers: measured 4e-2 relative error at layer 1 vs 4e-3 with per-layer scales).
 // Conversions saturate instead of producing inf; the weight gradients accumulate in fp32 and are
@@ -97,6 +98,7 @@ struct CompBwdParams {
   float* dsigma;
   float* dprergb;
   unsigned* amax_bits;      // [2]: max |d sigma|, max |d rgb_pre| as float bits (scale selection) or null
+  unsigned* tile_amax;      // [n_pad / 128][2]: the same two maxima per 128-sample tile (zero on entry)
 };
 
 __global__ void __launch_bounds__(128) composite_bwd_kernel(const CompBwdParams p) {
@@ -196,22 +198,36 @@ __global__ void __launch_bounds__(128) composite_bwd_kernel(const CompBwdParams 
     }
     if (lane == 0 && amax > 0.f && amax < 3e38f) atomicMax(p.amax_bits, __float_as_uint(amax));
     if (lane == 0 && amax_rgb > 0.f && amax_rgb < 3e38f) atomicMax(p.amax_bits + 1, __float_as_uint(amax_rgb));
+    // every tile this ray's samples fall in (non-negative floats order like their bits: deterministic)
+    if (p.tile_amax != nullptr && ray < p.n_rays && lane < 2) {
+      const float v = fminf(lane ? amax_rgb : amax, 3e38f);
+      if (v > 0.f)
+        for (long long t = (ray * S) >> 7; t <= (ray * S + S - 1) >> 7; ++t) atomicMax(p.tile_amax + 2 * t + lane, __float_as_uint(v));
+    }
   }
 }
 
 // Per-pass, per-level scales (see the header comment).  Level v: 0 = dd, v = 1..8 = dpre_{9-v}.
-//   phase 0 (before head_bwd / the probe): every level gets the level-0 scale
-//            2^floor(log2(64 / max(|d rgb_pre|_max wmax_rgb, |d sigma|_max wmax_sigma)))
-//   phase 1 (after the probe pass): levels 1..8 from the probe's per-level maxima (true, un-scaled
-//            values), clamped to [2^-12, 2^40] x level 0; a level the probe saw nothing in keeps its
-//            predecessor's scale.  Resets the statistics for the next step.
+//   phase 0 (before head_bwd / the probe): level 0 gets s0 = 2^floor(log2(64 / B0)) with the batch-wide bound
+//            B0 = max(|d rgb_pre|_max wmax_rgb, |d sigma|_max wmax_sigma) >= |dd|, |d sigma w_sigma|; levels
+//            1..8 get s0 / 16 for the probe pass (room for a growth of 2^14 through the chain before the probe's
+//            own conversions saturate).  Stores wmax_rgb / wmax_sigma for the probe's per-tile bounds.
+//   phase 1 (after the probe pass): the probe measured, per level, the growth factor g_v = max over the probed
+//            tiles of (largest |value| of the level in the tile) / (the tile's own level-0 bound).  The chain is
+//            linear in its level-0 input, so g_v does not depend on how large a tile's gradients are, and
+//            B0 g_v bounds level v of every probed tile: s_v = s0 2^-ceil(log2 g_v) maps that bound to <= 64.
+//            Clamped to [2^-40, 2^40] x s0; a level the probe saw nothing in keeps its predecessor's scale.
+//            Resets the statistics for the next step.
 constexpr int kLevels = 9;
+constexpr float kProbeLevelScale = 0.0625f;
 struct ScaleParams {
   int n_pass, phase;
   unsigned* amax;            // [2 passes][2]: |d sigma|, |d rgb_pre| maxima (float bits)
-  unsigned* lamax;           // [2 passes][kLevels] probe maxima (float bits)
+  unsigned* lamax;           // [2 passes][kLevels] probe growth factors (float bits)
   float* lscale;             // [2][kLevels]
   float* linv;               // [2][kLevels]
+  float* wnorm;              // [2 passes][2]: wmax_rgb, wmax_sigma
+  unsigned* saturated;       // [2 passes]: fp16 gradient elements the chain clipped (reset in phase 0)
   const float* w_rgb[2];     // live fp32 (3,128)
   const float* w_sigma[2];   // live fp32 (256)
 };
@@ -234,21 +250,25 @@ __global__ void __launch_bounds__(128) bwd_scale_kernel(const ScaleParams p) {
           const float bound = fmaxf(__uint_as_float(p.amax[2 * ps + 1]) * red[0][0], __uint_as_float(p.amax[2 * ps]) * red[1][0]);
           if (bound > 0.f) s = exp2f(floorf(log2f(64.f / bound)));
           s = fminf(fmaxf(s, 1e-30f), 1e30f);
+          if (t > 0) s *= kProbeLevelScale;
         }
         p.lscale[ps * kLevels + t] = s;
         p.linv[ps * kLevels + t] = 1.f / s;
         p.lamax[ps * kLevels + t] = 0u;
       }
+      if (t < 2) p.wnorm[2 * ps + t] = red[t][0];
+      if (t == 0) p.saturated[ps] = 0u;
       __syncthreads();
       if (t < 2) p.amax[2 * ps + t] = 0u;
     } else if (t == 0 && !kBwdBf16) {
       const float s0 = p.lscale[ps * kLevels];
       float prev = s0;
       for (int v = 1; v < kLevels; ++v) {
-        const float am = __uint_as_float(p.lamax[ps * kLevels + v]);
+        const float g = __uint_as_float(p.lamax[ps * kLevels + v]);
         float s = prev;
-        if (am > 0.f) s = exp2f(floorf(log2f(64.f / am)));
-        s = fminf(fmaxf(s, s0 * 2.44140625e-4f), s0 * 1.0995116e12f);
+        if (g > 0.f) s = s0 * exp2f(-ceilf(log2f(g)));
+        s = fminf(fmaxf(s, s0 * 9.094947e-13f), s0 * 1.0995116e12f);
+        s = fminf(fmaxf(s, 1e-30f), 1e30f);
         p.lscale[ps * kLevels + v] = s;
         p.linv[ps * kLevels + v] = 1.f / s;
         p.lamax[ps * kLevels + v] = 0u;
@@ -458,11 +478,43 @@ struct ChainParams {
   PassBufs pass[2];
   const uint8_t* net[2];      // packed images (backward region at kOffBwd, w_sigma in the fp32 region)
   int n_pass;
-  long long tiles[2];         // 128-sample tiles per pass (probe mode: the first tiles only)
+  long long tiles[2];         // 128-sample tiles per pass (probe mode: the number of probed tiles P)
+  long long pass_tiles[2];    // all 128-sample tiles of each pass
   const float* lscale;        // [2][kLevels] per-level scales (bwd_scale_kernel)
-  unsigned* lamax;            // probe mode: [2][kLevels] maxima of the un-scaled values per level
+  unsigned* lamax;            // probe mode: [2][kLevels] growth factors per level
+  unsigned* tile_amax[2];     // [pass_tiles][2] per-tile |d sigma|, |d rgb_pre| maxima (composite_bwd_kernel);
+                              // the probe reads them, the real pass zeroes them for the next step
+  const float* wnorm;         // [2][2] wmax_rgb, wmax_sigma (bwd_scale_kernel phase 0)
+  unsigned* saturated;        // real pass: [2] count of fp16 gradient elements at the fp16 limit (or NaN)
   int* status;
 };
+
+// The level-0 bound of one tile: the batch-wide bound of bwd_scale_kernel restricted to the tile.
+__device__ __forceinline__ float tile_bound(const ChainParams& p, int ps, long long tile) {
+  const unsigned* ta = p.tile_amax[ps] + 2 * tile;
+  return fmaxf(__uint_as_float(ta[1]) * p.wnorm[2 * ps], __uint_as_float(ta[0]) * p.wnorm[2 * ps + 1]);
+}
+
+// Probe mode: CTA c of a pass owns the tiles c, c + P, c + 2P, ... of that pass and probes the one with the
+// largest level-0 bound (the first on ties), so the batch's largest gradients are always probed.  Called by
+// whole warps: the lanes scan the candidates in parallel, every lane gets the same answer.
+__device__ __forceinline__ long long probe_tile(const ChainParams& p, int ps, long long cls, float* bound) {
+  const int lane = threadIdx.x & 31;
+  long long best = cls;
+  float bb = -1.f;
+  for (long long t = cls + lane * p.tiles[ps]; t < p.pass_tiles[ps]; t += 32 * p.tiles[ps]) {
+    const float b = tile_bound(p, ps, t);
+    if (b > bb) { bb = b; best = t; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ob = __shfl_xor_sync(0xffffffffu, bb, o);
+    const long long ot = __shfl_xor_sync(0xffffffffu, best, o);
+    if (ob > bb || (ob == bb && ot < best)) { bb = ob; best = ot; }
+  }
+  *bound = bb;
+  return best;
+}
 
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
   uint32_t d;
@@ -486,6 +538,7 @@ struct ChainEpi {
 //   kFirst: add the rank-1 sigma-head term;  kStore: hand the result to the next step (TMEM A operand)
 //   ratio = scale of the produced level / scale of the consumed level (a power of two)
 //   kProbe: no HBM stores; returns the largest |value| (in units of the produced level's scale)
+//   sat (real pass): incremented by the number of stored elements at the fp16 limit (satfinite clipped them) or NaN
 //   mw: this step's 64 ReLU sign bits (loaded one step earlier); next_mask: where the NEXT step's bits are (or null).
 //   The load is issued here, as soon as the accumulator is drained, and first used one step later: its HBM / L2
 //   latency hides behind this step's conversion and staging (it used to be issued at the top of the step it was
@@ -493,7 +546,7 @@ struct ChainEpi {
 //   d_ready wait of every step).
 template <bool kFirst, bool kStore, bool kProbe>
 __device__ __forceinline__ float epi_chain_step(ChainEpi& c, int out_idx, uint2& mw, const uint2* __restrict__ next_mask,
-                                                float dsig, const float* wsig, float ratio) {
+                                                float dsig, const float* wsig, float ratio, unsigned& sat) {
   // after << i the sign flag of pair i of K block kb sits in the top bit of byte 3 - kb (even elements in ylo, odd in yhi)
   uint32_t ylo[8], yhi[8];
 #pragma unroll
@@ -515,6 +568,7 @@ __device__ __forceinline__ float epi_chain_step(ChainEpi& c, int out_idx, uint2&
   uint8_t* out = c.dpre + static_cast<long long>(out_idx) * c.n_pad * 512 + (c.g0 & 63) * 128;
   const unsigned long long chunk = static_cast<unsigned long long>(c.g0 >> 6);
   uint32_t hs[4][8];
+  __half2 hmax = __float2half2_rn(0.f);      // per-half maximum of |h|, NaN-propagating (real pass)
 #pragma unroll
   for (int kb = 0; kb < 4; ++kb) {
     const int n0 = kb * 64 + c.part * 16;
@@ -537,6 +591,8 @@ __device__ __forceinline__ float epi_chain_step(ChainEpi& c, int out_idx, uint2&
       if (kProbe) {
         if (keep & 0xFFFFu) vmax = fmaxf(vmax, fabsf(a));
         if (keep >> 16) vmax = fmaxf(vmax, fabsf(b));
+      } else if (!kBwdBf16) {
+        hmax = __hmax2_nan(hmax, __habs2(*reinterpret_cast<const __half2*>(&h[i])));
       }
     }
     if (kStore) {
@@ -549,6 +605,12 @@ __device__ __forceinline__ float epi_chain_step(ChainEpi& c, int out_idx, uint2&
   }
   // the HBM copy for the wgrad kernel goes out after the hand-over, behind the next step's MMAs:
   // line-coalesced, staged per 32-row group, one 4 KiB bulk store each (mlp_engine.cuh stage_store)
+  if (!kProbe && !kBwdBf16 && __vcmpgeu2(*reinterpret_cast<const uint32_t*>(&hmax) & 0x7FFF7FFFu, 0x7BFF7BFFu) != 0u) {   // rare: count them
+#pragma unroll
+    for (int kb = 0; kb < 4; ++kb)
+#pragma unroll
+      for (int i = 0; i < 8; ++i) sat += __popc(__vcmpgeu2(hs[kb][i] & 0x7FFF7FFFu, 0x7BFF7BFFu)) >> 4;
+  }
   if (!kProbe) {
 #pragma unroll
     for (int kb = 0; kb < 4; ++kb)
@@ -583,6 +645,13 @@ __global__ void __launch_bounds__(kThreads, 1) chain_bwd_kernel(const ChainParam
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long total = p.tiles[0] + (p.n_pass > 1 ? p.tiles[1] : 0);
   const uint32_t idesc = make_idesc_f16(256) | (kBwdFmt << 7) | (kBwdFmt << 10);
+  // probe mode: one tile per CTA (grid = total), chosen by probe_tile
+  float probe_bound = 0.f;
+  long long probe_t = 0;
+  if (kProbe) {
+    const int ps = (blockIdx.x >= p.tiles[0]) ? 1 : 0;
+    probe_t = probe_tile(p, ps, blockIdx.x - (ps ? p.tiles[0] : 0), &probe_bound);
+  }
 
   if (warp == kProducerWarp) {
     if (lane == 0) {
@@ -590,7 +659,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_bwd_kernel(const ChainParam
       int it = 0;
       for (long long t = blockIdx.x; t < total; t += gridDim.x, ++it) {
         const int ps = (t >= p.tiles[0]) ? 1 : 0;
-        const long long tile = t - (ps ? p.tiles[0] : 0);
+        const long long tile = kProbe ? probe_t : t - (ps ? p.tiles[0] : 0);
         const int b = it & 1;
         // the dd tile: rows 0..63 and 64..127 of column block kb are two 8 KiB blocks of the tiled array
         mbar_wait(smem_u32(&sc->a0_empty[b]), ((it >> 1) & 1) ^ 1, 31);
@@ -684,13 +753,16 @@ __global__ void __launch_bounds__(kThreads, 1) chain_bwd_kernel(const ChainParam
     __syncwarp();
     if (lane == 0) mbar_arrive(smem_u32(&bars->d_free));
     uint2 mw = make_uint2(0u, 0u);      // ReLU sign bits of the step about to run (software-pipelined loads)
-    float amx[2][8];      // probe mode only: per pass and level, in un-scaled units
+    float amx[2][8];      // probe mode only: per pass and level, largest |value| over the tile's level-0 bound
 #pragma unroll
     for (int i = 0; i < 8; ++i) { amx[0][i] = 0.f; amx[1][i] = 0.f; }
+    unsigned sat[2] = {0u, 0u};
+    const float per_bound = (kProbe && probe_bound > 0.f) ? 1.f / probe_bound : 0.f;
     for (long long t = blockIdx.x; t < total; t += gridDim.x) {
       const int ps = (t >= p.tiles[0]) ? 1 : 0;
-      const long long tile = t - (ps ? p.tiles[0] : 0);
+      const long long tile = kProbe ? probe_t : t - (ps ? p.tiles[0] : 0);
       const PassBufs& pb = p.pass[ps];
+      if (!kProbe && warp == 0 && lane < 2) p.tile_amax[ps][2 * tile + lane] = 0u;     // read by this step's probe only
       c.dpre = pb.dpre;
       c.n_pad = pb.n_pad;
       c.g = tile * 128 + c.row;
@@ -704,14 +776,14 @@ __global__ void __launch_bounds__(kThreads, 1) chain_bwd_kernel(const ChainParam
         return q.mask + (static_cast<long long>(idx) * q.n_pad + g) * 4 + c.part;
       };
       if (t == static_cast<long long>(blockIdx.x)) mw = __ldg(mask_at(pb, c.g, 7));      // first tile: not prefetched
-      float m = epi_chain_step<true, true, kProbe>(c, 7, mw, mask_at(pb, c.g, 6), dsig, wsig, sc_out / sc_in);
-      if (kProbe) amx[ps][0] = fmaxf(amx[ps][0], m / sc_out);
+      float m = epi_chain_step<true, true, kProbe>(c, 7, mw, mask_at(pb, c.g, 6), dsig, wsig, sc_out / sc_in, sat[ps]);
+      if (kProbe) amx[ps][0] = fmaxf(amx[ps][0], m / sc_out * per_bound);
 #pragma unroll 1
       for (int s = 1; s < 7; ++s) {
         sc_in = sc_out;
         sc_out = ls[s + 1];
-        m = epi_chain_step<false, true, kProbe>(c, 7 - s, mw, mask_at(pb, c.g, 6 - s), 0.f, nullptr, sc_out / sc_in);
-        if (kProbe) amx[ps][s] = fmaxf(amx[ps][s], m / sc_out);
+        m = epi_chain_step<false, true, kProbe>(c, 7 - s, mw, mask_at(pb, c.g, 6 - s), 0.f, nullptr, sc_out / sc_in, sat[ps]);
+        if (kProbe) amx[ps][s] = fmaxf(amx[ps][s], m / sc_out * per_bound);
       }
       sc_in = sc_out;
       sc_out = ls[8];
@@ -725,10 +797,19 @@ __global__ void __launch_bounds__(kThreads, 1) chain_bwd_kernel(const ChainParam
           nxt = mask_at(p.pass[ps2], tile2 * 128 + c.row, 7);
         }
       }
-      m = epi_chain_step<false, false, kProbe>(c, 0, mw, nxt, 0.f, nullptr, sc_out / sc_in);
-      if (kProbe) amx[ps][7] = fmaxf(amx[ps][7], m / sc_out);
+      m = epi_chain_step<false, false, kProbe>(c, 0, mw, nxt, 0.f, nullptr, sc_out / sc_in, sat[ps]);
+      if (kProbe) amx[ps][7] = fmaxf(amx[ps][7], m / sc_out * per_bound);
     }
-    if (!kProbe) bulk_wait_all();
+    if (!kProbe) {
+      bulk_wait_all();
+#pragma unroll
+      for (int ps = 0; ps < 2; ++ps) {
+        unsigned v = sat[ps];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0 && v != 0u) atomicAdd(p.saturated + ps, v);
+      }
+    }
     if (kProbe) {
 #pragma unroll
       for (int ps = 0; ps < 2; ++ps)

@@ -183,6 +183,9 @@ struct TrainLayout {
   float* linv;                    // [2][kLevels] their inverses
   unsigned* lamax;                // [2][kLevels] probe statistics
   unsigned* amax;                 // [2][2] max |d sigma|, |d rgb_pre| per pass
+  unsigned* tile_amax[2];         // [n_pad / 128][2] the same maxima per 128-sample tile
+  float* wnorm;                   // [2][2] weight norms of the level-0 bound
+  unsigned* saturated;            // [2] fp16 gradient elements the last backward's chain clipped
   float* loss_part;               // [max CTAs][2]
   unsigned* loss_counter;
   size_t bytes;
@@ -243,6 +246,10 @@ void make_train_layout(TrainLayout* L, uint8_t* base, int64_t n_rays, int n_samp
   L->linv = reinterpret_cast<float*>(take(2 * kLevels * 4));
   L->lamax = reinterpret_cast<unsigned*>(take(2 * kLevels * 4));
   L->amax = reinterpret_cast<unsigned*>(take(16));
+  for (int ps = 0; ps < 2; ++ps)
+    L->tile_amax[ps] = ps < L->n_pass ? reinterpret_cast<unsigned*>(take(static_cast<size_t>(L->pass[ps].n_pad / 128) * 8)) : nullptr;
+  L->wnorm = reinterpret_cast<float*>(take(16));
+  L->saturated = reinterpret_cast<unsigned*>(take(8));
   L->loss_part = reinterpret_cast<float*>(take(1024 * 2 * 4));
   L->loss_counter = reinterpret_cast<unsigned*>(take(16));
   L->bytes = off;
@@ -932,12 +939,14 @@ int nerfb200_render_backward(const nerfb200_backward_args* b, void* stream_v) {
     cp.rgb_out = rgb_out[ps]; cp.target = b->target; cp.loss_grad = b->loss_grad;
     cp.dsigma = L.pass[ps].dsigma; cp.dprergb = L.pass[ps].dprergb;
     cp.amax_bits = L.amax + 2 * ps;
+    cp.tile_amax = L.tile_amax[ps];
     composite_bwd_kernel<<<(L.n_rays + 3) / 4, 128, 0, stream>>>(cp);
     g_launches++;
   }
   ScaleParams sp;
   sp.n_pass = L.n_pass; sp.phase = 0;
   sp.amax = L.amax; sp.lamax = L.lamax; sp.lscale = L.lscale; sp.linv = L.linv;
+  sp.wnorm = L.wnorm; sp.saturated = L.saturated;
   for (int ps = 0; ps < 2; ++ps) {
     const int q = ps < L.n_pass ? ps : 0;
     sp.w_rgb[ps] = params[q][22];
@@ -966,7 +975,8 @@ int nerfb200_render_backward(const nerfb200_backward_args* b, void* stream_v) {
     dir_grad_kernel<<<dim3(kDirSlices, L.n_pass), 128, 0, stream>>>(dp);
     g_launches++;
   }
-  // 3. dgrad chain (tcgen05): a probe pass over one tile per SM picks the per-layer scales, then the real pass
+  // 3. dgrad chain (tcgen05): a probe pass over one tile per SM (the largest of its stride class) measures the
+  //    per-layer growth factors that pick the per-layer scales, then the real pass
   {
     ChainParams cp;
     cp.n_pass = L.n_pass;
@@ -977,6 +987,10 @@ int nerfb200_render_backward(const nerfb200_backward_args* b, void* stream_v) {
     cp.lamax = L.lamax;
     cp.status = d->status;
     const long long t0 = L.pass[0].n_pad / 128, t1 = fine ? L.pass[1].n_pad / 128 : 0;
+    cp.pass_tiles[0] = t0; cp.pass_tiles[1] = t1;
+    cp.tile_amax[0] = L.tile_amax[0]; cp.tile_amax[1] = L.tile_amax[1];
+    cp.wnorm = L.wnorm;
+    cp.saturated = L.saturated;
     if (!kBwdBf16) {
       const long long half = (d->sm_count + 1) / 2;
       cp.tiles[0] = fine ? (t0 < half ? t0 : half) : (t0 < d->sm_count ? t0 : d->sm_count);
@@ -1049,6 +1063,22 @@ int nerfb200_render_backward(const nerfb200_backward_args* b, void* stream_v) {
   unfold_kernel<<<dim3((128 * 256 + (256 * 256 + 256 + 31) / 32 + 7) / 8, L.n_pass), 256, 0, stream>>>(up);
   g_launches++;
   CUDA_TRY(cudaGetLastError(), "render_backward launches");
+  return 0;
+}
+
+int nerfb200_train_saturation(const void* workspace, int64_t n_rays, int32_t n_samples, int32_t n_importance,
+                              uint32_t* out, void* stream_v) {
+  if (!workspace || !out || n_rays <= 0 || n_samples <= 0 || n_importance < 0)
+    return fail(NERFB200_EINVAL, "train_saturation: bad argument%s");
+  DeviceInfo* d = nullptr;
+  int rc = device_info(&d);
+  if (rc) return rc;
+  TrainLayout L;
+  make_train_layout(&L, static_cast<uint8_t*>(const_cast<void*>(workspace)), n_rays, n_samples, n_importance, d->sm_count);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  CUDA_TRY(cudaMemcpyAsync(out, L.saturated, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream), "saturation copy");
+  CUDA_TRY(cudaStreamSynchronize(stream), "saturation sync");
+  if (L.n_pass < 2) out[1] = 0;
   return 0;
 }
 

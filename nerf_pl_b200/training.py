@@ -17,6 +17,7 @@ The sampling of the fine depths carries no gradient (models/rendering.py:225-227
 from __future__ import annotations
 
 import ctypes
+import weakref
 from typing import Dict, List, Optional
 
 import torch
@@ -32,7 +33,8 @@ def _ptr(t: Optional[torch.Tensor]):
 class TrainWorkspace:
     """Device workspace of one (device, n_rays, N_samples, N_importance) shape, reused across steps.
     ``busy`` is set between a forward and its backward so that a second forward (gradient
-    accumulation over several batches) gets its own buffer."""
+    accumulation over several batches) gets its own buffer.  It is cleared by the backward, or when
+    the forward's autograd graph is freed without one (a skipped step, a forward under grad for logging)."""
 
     _pool: Dict[tuple, List["TrainWorkspace"]] = {}
 
@@ -46,6 +48,8 @@ class TrainWorkspace:
         self.raw = raw
         self.buf = raw[off:off + self.bytes]
         self.busy = False
+        self.shape = (n, S_c, K)
+        self.device = dev
         with torch.cuda.device(dev):
             _lib.check(lib.nerfb200_train_workspace_init(self.buf.data_ptr(), self.bytes, n, S_c, K, _stream_ptr()),
                        "nerfb200_train_workspace_init")
@@ -62,6 +66,18 @@ class TrainWorkspace:
         ws.busy = True
         free.append(ws)
         return ws
+
+    def release(self) -> None:
+        self.busy = False
+
+    def saturated(self):
+        """(coarse, fine) count of fp16 gradient elements the last backward on this workspace clipped at
+        the fp16 limit or stored as NaN (``nerfb200_train_saturation``).  Synchronises the current stream."""
+        out = (ctypes.c_uint32 * 2)()
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.load().nerfb200_train_saturation(self.buf.data_ptr(), *self.shape, out, _stream_ptr()),
+                       "nerfb200_train_saturation")
+        return int(out[0]), int(out[1])
 
     @classmethod
     def clear(cls) -> None:
@@ -108,7 +124,9 @@ class FusedRenderFunction(torch.autograd.Function):
         with torch.cuda.device(dev):
             _lib.check(lib.nerfb200_render_rays(ctypes.byref(args), _stream_ptr()), "nerfb200_render_rays")
         ctx.cfg = cfg
-        ctx.keep = (rays, pr, nc, ur, nf, target, out, blob_c, blob_f, ws)
+        # detached views of the outputs: the outputs themselves would close a reference cycle through ctx
+        ctx.keep = (rays, pr, nc, ur, nf, target, [o.detach() for o in out], blob_c, blob_f, ws)
+        ctx.release_ws = weakref.finalize(ctx, ws.release)      # also runs if the graph dies without a backward
         ctx.n_params = len(params)
         ctx.save_for_backward(*params)
         ctx.set_materialize_grads(False)
@@ -159,7 +177,7 @@ class FusedRenderFunction(torch.autograd.Function):
             grads_coarse=gc, grads_fine=gf)
         with torch.cuda.device(dev):
             _lib.check(lib.nerfb200_render_backward(ctypes.byref(bargs), _stream_ptr()), "nerfb200_render_backward")
-        ws.busy = False
+        ctx.release_ws()
         ctx.keep = None
         if K == 0:
             grads = grads[:24] + [None] * (ctx.n_params - 24)
